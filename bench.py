@@ -4,6 +4,7 @@
   python bench.py --gpus 1 --steps 5 --warmup 3
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
   python bench.py --impl reference ...      # the reference's CPU path (C restatement in oracle/) on the host cores
+  python bench.py --dump-outputs DIR ...    # also write the compressed stream of the last timed step to DIR (dump_outputs)
 
 Workload (N = 1): BASELINE.json configs[1] -- 100 MB of enwik8-shaped synthetic text, quality 5, lgwin 22.
 A step = one pass of the compression hot path over that input.  For N > 1 the stream is N x 100 MB, sharded with the
@@ -35,6 +36,24 @@ CHUNK_BYTES = 24 << 20       # one k_match launch per chunk (csrc/bro_parse.cuh 
 # capture summarised in profiles/ (None until a capture of the current kernel exists)
 NCU_MATCH_DRAM_BYTES_PER_LAUNCH = 774_424_320 + 669_327_104
 NCU_MATCH_SOURCE = "profiles/r02x_ncu_q5.txt (ncu --set full, one k_match_shallow<16> launch: 29.4 M sorted entries, 25.2 M payload positions)"
+DUMP_MAX_BYTES = 8 << 20  # stream bytes --dump-outputs writes over all ranks: 32 MiB as float32, within its 64 MB budget
+
+
+def dump_outputs(out_dir, comp, rank=0, world=1):
+    """--dump-outputs: what a caller of the timed path receives -- the compressed stream -- as float32 byte values
+    (`compressed.npy`) and its length (`compressed_size.npy`, float64); with world > 1 every rank writes its own shard's
+    stream under a `rank<r>_` prefix.  Each rank keeps at most DUMP_MAX_BYTES // world bytes, so the whole dump stays within
+    DUMP_MAX_BYTES; a longer stream is represented by its bytes at that many positions drawn with a fixed seed, in stream
+    order.  The positions depend on the stream length only, so two builds that produce the same stream write the same arrays."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    prefix = "rank%d_" % rank if world > 1 else ""
+    limit = DUMP_MAX_BYTES // world
+    b = comp.cpu().numpy()
+    np.save(os.path.join(out_dir, prefix + "compressed_size.npy"), np.array([b.size], dtype=np.float64))
+    if b.size > limit:
+        b = b[np.sort(np.random.default_rng(0).choice(b.size, limit, replace=False))]
+    np.save(os.path.join(out_dir, prefix + "compressed.npy"), b.astype(np.float32))
 
 
 def load_peaks():
@@ -158,7 +177,12 @@ def main():
     # "text5" = BASELINE configs[1] (the metric's configuration, the default); "json9" = BASELINE configs[3]: JSON logs, quality 9,
     # 512 MiB per GPU (4 GiB over 8 GPUs), the compress_multi split across ranks
     ap.add_argument("--config", default="text5", choices=["text5", "json9"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the compressed stream of the last timed step to DIR as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the device path; --impl reference has no timed output to dump")
     if args.config == "json9":
         if args.bytes == WORKLOAD_BYTES:
             args.bytes = 512 << 20
@@ -323,12 +347,14 @@ def main():
     launches = 0
     ev[0].record()
     for _ in range(args.steps):
-        step_resident()
+        n_last = step_resident()
         launches += enc.timings()[1]
     ev[1].record()
     barrier()
     wall = ev[0].elapsed_time(ev[1]) * 1e-3
     clocks = sampler.stop()
+    if args.dump_outputs:  # before the loops below reuse d_out
+        dump_outputs(args.dump_outputs, d_out[:n_last], rank, world)
     # ---- e2e: host buffers through the C ABI ----
     for _ in range(2):
         step_e2e()
